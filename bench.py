@@ -7,7 +7,11 @@ gate/up+SiLU*mul, down} + lm_head = 6.607e9 Q4_0 weights = 3.716 GB of packed by
 the device exactly as ne_compute_forward_mul_mat_q_f32 does, all captured in one CUDA graph.  Synthetic data:
 W ~ N(0, 0.02^2) (torch.manual_seed(1234)), quantised to Q4_0 on the device by the library's own quantiser.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--fmt q4_0|int4g128]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--fmt q4_0|int4g128] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed path computed in its last timed step, as float32 DIR/<name>.npy: the logits and the
+outputs of the last layer's matmul nodes (every layer writes the same buffers).  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 
 Keys beyond the base contract: roofline{} (dominant kernel = the streaming GEMV, timed live with CUDA events on the
 launching stream), cpu_baseline{} (the reference's own ggml Q4_0 x Q8_0 code, oracle/_ref, timed on this box's host cores
@@ -40,6 +44,15 @@ try:
         METRIC = json.load(_f).get("metric", METRIC)
 except (OSError, ValueError):
     pass
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> array; written as float32 .npy files under path (at most 64 MB in all)"""
+    os.makedirs(path, exist_ok=True)
+    arrays = {name: np.ascontiguousarray(a, dtype=np.float32) for name, a in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def shapes():
@@ -171,15 +184,18 @@ class CpuReference:
         self.threads = host_threads()
 
     def token(self, n_layers=N_LAYER):
-        """all matmuls of one decode token (7 per layer, unfused, as the ggml path runs them) + lm_head"""
+        """all matmuls of one decode token (7 per layer, unfused, as the ggml path runs them) + lm_head; self.last keeps the
+        last layer's outputs and the logits"""
         mm = lambda wq, a: self.o.mul_mat_q4_0_f32(wq, a, self.impl, nth=self.threads)
+        out = {}
         for l in range(n_layers):
             ws = self.layers[l % len(self.layers)]
             for name in ("wq", "wk", "wv", "wo", "w1", "w3"):
-                mm(ws[name], self.x)
-            mm(ws["w2"], self.h)
+                out["last_layer_" + name] = mm(ws[name], self.x)
+            out["last_layer_w2"] = mm(ws["w2"], self.h)
         if n_layers == N_LAYER:
-            mm(self.lm_head, self.x)
+            out["logits"] = mm(self.lm_head, self.x)
+        self.last = out
 
     def time_tokens(self, tokens, warmup=1):
         for _ in range(warmup):
@@ -197,6 +213,8 @@ def run_reference(args):
         return
     ref = CpuReference()
     tps, spt = ref.time_tokens(args.steps, max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ref.last)
     line = {
         "impl": "reference", "metric": METRIC, "value": tps, "unit": "tokens/s", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": spt * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -463,6 +481,9 @@ def run_ours(args):
         sampler.start()
     ms_perop = timed(run_step, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:  # before any other leg reuses these buffers
+        dump_outputs(args.dump_outputs, {"last_layer_qkv": qkv.cpu().numpy(), "last_layer_o": o.cpu().numpy(),
+                                         "last_layer_ffn": ffn.cpu().numpy(), "logits": logits.cpu().numpy()})
     # a leg of at least one second of back-to-back steps: sustained clocks / power rather than a 20 ms burst
     sus_steps = max(args.steps, int(1.05 / (ms_perop * 1e-3)))
     ms_sus = timed(run_step, sus_steps, 3)
@@ -819,7 +840,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 500; 20 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--fmt", default="q4_0", choices=["q4_0", "int4g128"])
@@ -833,10 +854,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="skip the BASELINE configs 2-4 legs")
     ap.add_argument("--skip-tp", action="store_true", help="N > 1: skip the Llama-2-70B tensor-parallel leg (config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 500
     if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 20
         run_reference(args)
     else:
         run_ours(args)

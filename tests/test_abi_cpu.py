@@ -132,23 +132,32 @@ def test_qpack_with_zero_points_and_gidx():
         assert np.array_equal(sh[b * g:(b + 1) * g], np.nonzero(g_idx == b)[0])
 
 
-@pytest.mark.skipif(oracle.ref_btla() is None, reason="oracle/_ref/libref_btla.so not built")
 def test_oracle_blob_layout_against_reference_kernels():
-    """pin oracle/btla_blob.py's interleave/compress against kernel_ref.h padding_interleave + compress_s8_s4"""
-    R = oracle.ref_btla()
+    """pin oracle/btla_blob.py's interleave/compress against kernel_ref.h padding_interleave + compress_s8_s4 (their answers for
+    these inputs: tests/golden/reference.npz)"""
+    from oracle import golden
     rng = np.random.default_rng(12)
     for (ntile, packrow, k, n) in [(48, 4, 64, 100), (48, 1, 40, 48), (24, 2, 64, 30), (48, 2, 96, 144)]:
         q = rng.integers(-8, 8, (k, n)).astype(np.int8)
         kpad = -(-k // packrow) * packrow
         npad = -(-n // ntile) * ntile
-        dst = np.zeros(kpad * npad, np.int8)
-        R.ref_btla_padding_interleave_s8(q.ctypes.data_as(C.c_void_p), dst.ctypes.data_as(C.c_void_p), k, n, kpad, npad, n,
-                                         kpad, ntile, packrow)
+
+        def interleave():
+            dst = np.zeros(kpad * npad, np.int8)
+            oracle.ref_btla().ref_btla_padding_interleave_s8(q.ctypes.data_as(C.c_void_p), dst.ctypes.data_as(C.c_void_p), k, n, kpad,
+                                                             npad, n, kpad, ntile, packrow)
+            return dst
+
+        def compress(dst):
+            packed = np.zeros(dst.size // 2, np.uint8)
+            oracle.ref_btla().ref_btla_compress_s8_s4(dst.ctypes.data_as(C.c_void_p), packed.ctypes.data_as(C.c_void_p),
+                                                      C.c_size_t(dst.size))
+            return packed
+
+        key = f"blob_layout[{ntile}-{packrow}-{k}-{n}]"
         mine = btla_blob.interleave(q, ntile, packrow, kpad, npad)
-        assert np.array_equal(dst, mine)
-        packed = np.zeros(dst.size // 2, np.uint8)
-        R.ref_btla_compress_s8_s4(dst.ctypes.data_as(C.c_void_p), packed.ctypes.data_as(C.c_void_p), C.c_size_t(dst.size))
-        assert np.array_equal(packed, btla_blob.compress_s4(mine))
+        golden.check(key + ".interleave", mine, interleave)
+        golden.check(key + ".compress_s4", btla_blob.compress_s4(mine), lambda: compress(interleave()))
 
 
 def test_packweight_copyattr_matches_direct_quantisation():

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 import oracle
@@ -12,9 +13,9 @@ import oracle
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_the_contract_line():
-    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
-                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+def test_reference_arm_prints_the_contract_line(tmp_path):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [ln for ln in p.stdout.strip().splitlines() if ln.startswith("{")]
     assert len(lines) == 1
@@ -28,6 +29,10 @@ def test_reference_arm_prints_the_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == ("reference" if oracle.ref_ggml() is not None else "port") and cb["cores"] >= 1 and cb["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    # --dump-outputs: the last timed token's matmul outputs, float32
+    logits = np.load(tmp_path / "out" / "logits.npy")
+    assert logits.dtype == np.float32 and logits.shape == (1, 32000) and np.isfinite(logits).all()
+    assert np.load(tmp_path / "out" / "last_layer_w2.npy").shape == (1, 4096)
 
 
 def test_default_arm_needs_a_gpu():

@@ -124,13 +124,7 @@ def _btla_oracle_mm(w_nk, g, asym, a):
     return oracle.btla_gemv_u8s8(a8, asc, azp, q, sc, zp, g)
 
 
-@pytest.mark.parametrize("g,alg,threads", [(32, "sym", 1), (128, "asym", 3)])
-def test_btla_experts_through_the_reference_engine_on_the_drop_ins(g, alg, threads):
-    """ne_graph_compute of the REFERENCE (linked against libns_b200.so) runs NE_OP_MUL_MAT_ID on BesTLA experts token by token
-    through bestla_f32f32_forward; ns_mul_mat_id groups the tokens.  Both must give the CPU oracle's numbers."""
-    Lns = oracle.ref_ne_ns()
-    if Lns is None:
-        pytest.skip("oracle/_ref/libref_ne_ns.so not built (needs /root/reference at build time)")
+def _btla_experts(g, alg):
     rng = np.random.default_rng(60 + g)
     n_as, n, k, m, n_used = 4, 256, 512, 9, 2
     w = [rng.normal(0, 1.0 / np.sqrt(k), (n, k)).astype(np.float32) for _ in range(n_as)]
@@ -138,10 +132,29 @@ def test_btla_experts_through_the_reference_engine_on_the_drop_ins(g, alg, threa
     a = rng.normal(0, 1, (m, k)).astype(np.float32)
     ids = rng.integers(0, n_as, (m, n_used)).astype(np.int32)
     want = np.stack([_btla_oracle_mm(w[int(ids[t, 1])], g, alg == "asym", a[t:t + 1])[0] for t in range(m)])
+    return blobs, a, ids, want
+
+
+@pytest.mark.parametrize("g,alg,threads", [(32, "sym", 1), (128, "asym", 3)])
+def test_btla_experts_through_the_reference_engine_on_the_drop_ins(g, alg, threads):
+    """ne_graph_compute of the REFERENCE (linked against libns_b200.so) runs NE_OP_MUL_MAT_ID on BesTLA experts token by token
+    through bestla_f32f32_forward: it must give the CPU oracle's numbers.  Runs where oracle/_ref was built with the reference."""
+    Lns = oracle.ref_ne_ns()
+    if Lns is None:
+        pytest.skip("oracle/_ref/libref_ne_ns.so not built (the reference's engine is not part of this repository)")
+    blobs, a, ids, want = _btla_experts(g, alg)
+    n, k = want.shape[1], a.shape[1]
     lc0 = ns.lib().ns_launch_count()
     eng = oracle.ref_mul_mat_id(Lns, blobs, oracle.NE_TYPE_BTLA, n, k, ids, 1, a, n_threads=threads)
     assert ns.lib().ns_launch_count() > lc0, "the reference engine did not reach the CUDA kernels"
     close(eng, want, 1e-4)
+
+
+@pytest.mark.parametrize("g,alg", [(32, "sym"), (128, "asym")])
+def test_btla_experts_grouped_by_ns_mul_mat_id(g, alg):
+    """ns_mul_mat_id groups the tokens by expert: it must give the CPU oracle's numbers for the selected expert of every token."""
+    blobs, a, ids, want = _btla_experts(g, alg)
+    m, n, k = a.shape[0], want.shape[1], a.shape[1]
     ws = [ns.Weight.from_blob(b) for b in blobs]
     ad = dev(a)
     out = torch.full((m, n), float("nan"), device="cuda")
@@ -151,9 +164,7 @@ def test_btla_experts_through_the_reference_engine_on_the_drop_ins(g, alg, threa
     close(out.cpu().numpy(), want, 1e-4)
 
 
-def test_ffn_id_against_the_reference_engine_and_the_oracle():
-    """ne_mul_id_ffn_silu: one decode token through the reference engine on the drop-ins (it reads ONE id for the whole node,
-    ne_layers.c:8062) and a 6-token batch with per-token experts through ns_ffn_id against per-token fused FFNs."""
+def _ffn_id_experts():
     rng = np.random.default_rng(71)
     n_as, k, fmid, g = 4, 256, 704, 128
     mk = lambda r, c: ns.np_bestla_quantize(rng.normal(0, 1.0 / np.sqrt(c), (r, c)).astype(np.float32), "int4", g, "sym", "fp32", "int8")
@@ -162,6 +173,11 @@ def test_ffn_id_against_the_reference_engine_and_the_oracle():
     m = 6
     x = rng.normal(0, 1, (m, k)).astype(np.float32)
     ids = rng.integers(0, n_as, (m, 2)).astype(np.int32)
+    return (gate, up, down), (wg, wu, wd), x, ids
+
+
+def _ffn_id(wg, wu, wd, x, ids):
+    m, k, fmid = x.shape[0], x.shape[1], wg[0].n
     xd = dev(x)
     tmp = torch.zeros(2 * m * fmid, device="cuda")
     out = torch.full((m, k), float("nan"), device="cuda")
@@ -177,8 +193,23 @@ def test_ffn_id_against_the_reference_engine_and_the_oracle():
         ns.ffn_silu(wg[e], wd[e], wu[e], xd[t:t + 1].data_ptr(), k, t1.data_ptr(), one.data_ptr(), k, 1)
         sync()
         close(got[t:t + 1], one.cpu().numpy(), 1e-4)
+    return got
+
+
+def test_ffn_id_against_per_token_fused_ffns():
+    """ne_mul_id_ffn_silu: a 6-token batch with per-token experts through ns_ffn_id against per-token fused FFNs."""
+    _, (wg, wu, wd), x, ids = _ffn_id_experts()
+    _ffn_id(wg, wu, wd, x, ids)
+
+
+def test_ffn_id_against_the_reference_engine_and_the_oracle():
+    """ne_mul_id_ffn_silu: one decode token through the reference engine on the drop-ins (it reads ONE id for the whole node,
+    ne_layers.c:8062) against ns_ffn_id.  Runs where oracle/_ref was built with the reference."""
     Lns = oracle.ref_ne_ns()
     if Lns is None:
-        pytest.skip("oracle/_ref/libref_ne_ns.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libref_ne_ns.so not built (the reference's engine is not part of this repository)")
+    (gate, up, down), (wg, wu, wd), x, ids = _ffn_id_experts()
+    got = _ffn_id(wg, wu, wd, x, ids)
+    k, fmid = x.shape[1], wg[0].n
     eng = oracle.ref_ffn_id_silu(Lns, gate, down, up, k, fmid, k, ids[:1], 1, x[:1], n_threads=2)
     close(eng, got[:1], 1e-4)

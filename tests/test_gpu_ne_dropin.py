@@ -21,7 +21,7 @@ def _need():
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     if oracle.ref_ne_ns() is None:
-        pytest.skip("oracle/_ref/libref_ne_ns.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libref_ne_ns.so not built (the reference's engine is not part of this repository)")
     ns.lib().bestla_init()
     yield
     ns.lib().ns_host_cache_clear()

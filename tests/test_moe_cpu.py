@@ -1,12 +1,14 @@
 """CPU side of the expert-indexed matmul (ne_mul_mat_id): the oracle restatement against the REFERENCE's own engine
-(ne_compute_forward_mul_mat_id_q_f32, core/ne_layers.c:7345-7498, run through ne_graph_compute) and against the committed
-golden fixture generated from it (tests/golden/make_golden_moe.py)."""
+(ne_compute_forward_mul_mat_id_q_f32, core/ne_layers.c:7345-7498, run through ne_graph_compute; its answers for these inputs
+are stored in tests/golden/reference.npz) and against the committed golden fixture generated from it
+(tests/golden/make_golden_moe.py)."""
 import os
 
 import numpy as np
 import pytest
 
 import oracle
+from oracle import golden
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -21,9 +23,6 @@ def test_restatement_matches_the_golden_fixture_bit_for_bit():
 
 @pytest.mark.parametrize("n_threads", [1, 3])
 def test_restatement_matches_the_reference_engine(n_threads):
-    L = oracle.ref_ne()
-    if L is None:
-        pytest.skip("oracle/_ref/libref_ne.so not built (needs /root/reference)")
     rng = np.random.default_rng(7 + n_threads)
     n_as, n, k, n_tok, n_used = 8, 64, 512, 11, 2
     rows = [oracle.quantize_q4_0(rng.normal(0, 0.02, (n, k)).astype(np.float32)) for _ in range(n_as)]
@@ -31,9 +30,9 @@ def test_restatement_matches_the_reference_engine(n_threads):
     ids = rng.integers(0, n_as, (n_tok, n_used)).astype(np.int32)
     ids[:3, 0] = 5  # a run of tokens on one expert and experts nobody picked
     for slot in range(n_used):
-        want = oracle.ref_mul_mat_id(L, rows, oracle.NE_TYPE_Q4_0, n, k, ids, slot, a, n_threads=n_threads)
         got = oracle.mul_mat_id_q4_0_f32(rows, ids, slot, a)
-        assert np.array_equal(got, want)
+        golden.check(f"mul_mat_id[{n_threads}].slot{slot}", got,
+                     lambda: oracle.ref_mul_mat_id(oracle.ref_ne(), rows, oracle.NE_TYPE_Q4_0, n, k, ids, slot, a, n_threads=n_threads))
 
 
 def test_host_side_grouping_of_tokens_by_expert():

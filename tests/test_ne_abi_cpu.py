@@ -1,15 +1,17 @@
 """include/ns_ne_abi.h restates struct ne_tensor / ne_compute_params and a few enum values of the reference's graph engine (the
-structs bestla_support / bestla_parallel_for receive).  Where /root/reference is present, compile both headers into one C file and
-let the compiler compare every offset, size and enum value; elsewhere check the committed numbers (taken from that compile)."""
+structs bestla_support / bestla_parallel_for receive).  Every offset, size and enum value of ns_ne_abi.h must equal the one the
+reference's core/ne.h gives; the reference's numbers (x86-64 LP64) are stored in tests/golden/reference.npz, recorded by compiling
+the same program against that header."""
 import ctypes as C
 import os
 import subprocess
 import tempfile
 
-import pytest
+import numpy as np
+
+from oracle import golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/neural_speed"
 
 FIELDS = ["type", "backend", "n_dims", "ne", "nb", "op", "is_param", "op_params", "grad", "src0", "src1", "opt", "n_tasks", "perf_runs",
           "perf_cycles", "perf_time_us", "data", "size", "name", "padding"]
@@ -26,24 +28,27 @@ ENUMS = {"NE_TYPE_F32": "NS_NE_TYPE_F32", "NE_TYPE_F16": "NS_NE_TYPE_F16", "NE_T
          "NE_MAX_OP_PARAMS": "NS_NE_MAX_OP_PARAMS"}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference headers not present on this box")
-def test_layout_matches_the_reference_header():
-    lines = ['#include <stddef.h>', '#include "core/ne.h"', '#include "ns_ne_abi.h"']
-    for f in FIELDS:
-        lines.append(f'_Static_assert(offsetof(struct ne_tensor, {f}) == offsetof(struct ns_ne_tensor, {f}), "ne_tensor.{f}");')
-    for f in PFIELDS:
-        lines.append(f'_Static_assert(offsetof(struct ne_compute_params, {f}) == offsetof(struct ns_ne_compute_params, {f}), "params.{f}");')
-    lines.append('_Static_assert(sizeof(struct ne_tensor) == sizeof(struct ns_ne_tensor), "sizeof ne_tensor");')
-    lines.append('_Static_assert(sizeof(struct ne_compute_params) == sizeof(struct ns_ne_compute_params), "sizeof params");')
-    for a, b in ENUMS.items():
-        lines.append(f'_Static_assert((int){a} == (int){b}, "{a}");')
-    lines.append("int main(void) { return 0; }")
+def _layout(header, tensor, params, enums, incs):
+    """offsets of FIELDS / PFIELDS, both sizeofs and the enum values, as one header declares them"""
+    vals = [f"offsetof(struct {tensor}, {f})" for f in FIELDS] + [f"offsetof(struct {params}, {f})" for f in PFIELDS]
+    vals += [f"sizeof(struct {tensor})", f"sizeof(struct {params})"] + [f"(long)({e})" for e in enums]
+    body = "".join(f'printf("%ld\\n", (long)({v}));' for v in vals)
     with tempfile.TemporaryDirectory() as d:
-        src = os.path.join(d, "chk.c")
-        open(src, "w").write("\n".join(lines))
-        r = subprocess.run(["gcc", "-std=c11", "-fsyntax-only", f"-I{REF}", f"-I{REF}/core", f"-I{ROOT}/include", src], capture_output=True,
-                           text=True)
+        src, exe = os.path.join(d, "layout.c"), os.path.join(d, "layout")
+        open(src, "w").write(f'#include <stdio.h>\n#include <stddef.h>\n#include "{header}"\nint main(void){{{body}return 0;}}\n')
+        r = subprocess.run(["gcc", "-std=c11", *[f"-I{i}" for i in incs], src, "-o", exe], capture_output=True, text=True)
         assert r.returncode == 0, r.stderr
+        out = subprocess.run([exe], capture_output=True, text=True, check=True).stdout.split()
+    return np.array([int(v) for v in out], np.int64)
+
+
+def test_layout_matches_the_reference_header():
+    def reference():
+        ref = os.path.join(golden.SOURCE, "neural_speed")
+        return _layout("core/ne.h", "ne_tensor", "ne_compute_params", list(ENUMS), [ref, f"{ref}/core"])
+
+    golden.check("ne_abi.layout", _layout("ns_ne_abi.h", "ns_ne_tensor", "ns_ne_compute_params", list(ENUMS.values()), [f"{ROOT}/include"]),
+                 reference)
 
 
 def test_committed_layout_numbers():

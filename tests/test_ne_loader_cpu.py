@@ -1,6 +1,7 @@
 """Reader for neural-speed's native `.bin` (NE / ggjt) model files.  The test file is written the way the reference's own
-converter writes it (convert/convert_quantized_llama.py:131-260): header and vocab in that order, tensor headers through the
-reference's `write_header` (convert/common.py:467) when /root/reference is importable."""
+converter writes it (convert/convert_quantized_llama.py:131-260): header and vocab in that order, tensor headers as the
+reference's `write_header` (convert/common.py:467) writes them -- the bytes it wrote for this file are stored in
+tests/golden/reference.npz -- or through a restatement of it."""
 import importlib.util
 import os
 import struct
@@ -10,17 +11,48 @@ import pytest
 
 import neural_speed_b200 as ns
 from neural_speed_b200 import ne_loader
+from oracle import golden
 
-REF_COMMON = "/root/reference/neural_speed/convert/common.py"
+
+class _Tap:
+    """the bytes a header writer leaves in the file, the alignment gap it seeks over included"""
+
+    def __init__(self, f):
+        self.f, self.data = f, bytearray()
+
+    def write(self, b):
+        self.data += b
+        return self.f.write(b)
+
+    def tell(self):
+        return self.f.tell()
+
+    def seek(self, pos):
+        self.data += bytes(pos - self.f.tell())
+        return self.f.seek(pos)
 
 
 def _ref_write_header():
-    if not os.path.exists(REF_COMMON):
-        return None
-    spec = importlib.util.spec_from_file_location("ref_common_ne", REF_COMMON)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m.write_header
+    """the reference's write_header, replaying the bytes it wrote for each tensor header of _write's file"""
+    def live():
+        spec = importlib.util.spec_from_file_location("ref_common_ne", os.path.join(golden.SOURCE, "neural_speed", "convert", "common.py"))
+        m = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(m)
+        return m.write_header
+
+    def write_header(f, shape, name, ftype):
+        def written():
+            tap = _Tap(f)
+            live()(tap, shape, name, ftype)
+            return np.frombuffer(bytes(tap.data), np.uint8)
+
+        key = f"ne_header[{f.tell()}].{name}"
+        if golden.recording():
+            golden.value(key, written)
+        else:
+            f.write(golden.value(key, None).tobytes())
+
+    return write_header
 
 
 def _own_write_header(f, shape, name, ftype):
@@ -84,8 +116,6 @@ def _write(path, write_header):
 @pytest.mark.parametrize("writer", ["reference", "own"])
 def test_parse_ne_llama_file_with_btla_blobs(tmp_path, writer):
     wh = _ref_write_header() if writer == "reference" else _own_write_header
-    if wh is None:
-        pytest.skip("/root/reference not present")
     path = str(tmp_path / "tiny.bin")
     ref, hp = _write(path, wh)
     raw_hp, vocab, special, tensors = ne_loader.read_file(path)
