@@ -325,6 +325,15 @@ NS_API int ns_llama_generate(ns_llama* ctx, int32_t first_token, int n_past, int
  * tokens instead: reference numerics for the whole prompt at about 1/6 of the prefill throughput. */
 NS_API int ns_llama_set_exact_prefill(ns_llama* ctx, int on);
 NS_API unsigned long long ns_llama_kv_bytes(const ns_llama* ctx);
+/* Test / debug surfaces: what one layer's attention saw and wrote, so that it can be checked against a reference outside
+ * the engine.  With a tap on `layer`, every eval (and every step of a one-token graph) copies, on the context's stream,
+ *   qkv_dst  <- the layer's q | k | v before RoPE: [m][n_embd] | [m][kvd] | [m][kvd] floats (kvd = n_head_kv * head size),
+ *   attn_dst <- the attention output [m][n_embd] floats,
+ * both device pointers.  An eval of more than max_rows tokens fails.  layer < 0 removes the tap.  Setting or removing a tap
+ * rebuilds the one-token graph; without a tap the enqueued work is unchanged. */
+NS_API int ns_llama_set_tap(ns_llama* ctx, int layer, float* qkv_dst, float* attn_dst, int max_rows);
+/* device pointers to the fp16 KV cache of `layer`: k and v are each [n_head_kv][n_ctx][head size] */
+NS_API int ns_llama_kv_cache(const ns_llama* ctx, int layer, const void** k, const void** v);
 
 /* ---- tensor-parallel exchange step over NVLink peer memory (SURVEY 8e) --------------------------------------------
  * One-shot sum all-reduce replacing reduce_add / ne_all_reduce (core/parallel_context.cpp:47, ne_layers.c:5466) for the

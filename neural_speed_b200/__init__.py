@@ -58,7 +58,7 @@ EXPORTS = [
     "ns_device_quantize_q4_0", "ns_device_quantize_act",
     "BTLAGemmPackBSize", "BTLAGemmQuantPackB", "BTLAGemmPackB", "BTLAGemmUnPackB", "ns_quantize_row_q4_0", "ns_split_weight_size", "ns_split_weight",
     "ns_llama_create", "ns_llama_free", "ns_llama_set_f32", "ns_llama_set_weight", "ns_llama_eval", "ns_llama_generate", "ns_llama_set_exact_prefill",
-    "ns_llama_kv_bytes",
+    "ns_llama_kv_bytes", "ns_llama_set_tap", "ns_llama_kv_cache",
     "ns_comm_handle_bytes", "ns_comm_create", "ns_comm_get_handle", "ns_comm_open_peers", "ns_comm_link_local", "ns_comm_all_reduce_f32",
     "ns_comm_status", "ns_comm_free",
 ]
@@ -180,6 +180,8 @@ def lib() -> C.CDLL:
     L.ns_llama_generate.argtypes = [vp, C.c_int32, i, i, vp]
     L.ns_llama_kv_bytes.restype = C.c_ulonglong
     L.ns_llama_kv_bytes.argtypes = [vp]
+    L.ns_llama_set_tap.argtypes = [vp, i, vp, vp, i]
+    L.ns_llama_kv_cache.argtypes = [vp, i, C.POINTER(vp), C.POINTER(vp)]
     L.ns_comm_handle_bytes.restype = sz
     L.ns_comm_create.restype = vp
     L.ns_comm_create.argtypes = [i, i, sz, vp]
@@ -482,6 +484,47 @@ class Llama:
 
     def kv_bytes(self) -> int:
         return int(lib().ns_llama_kv_bytes(self.h))
+
+    def _dims(self):
+        hd = self.hp.n_embd // self.hp.n_head
+        return self.hp.n_embd, hd * self.hp.n_head_kv, hd
+
+    def set_tap(self, layer: int, max_rows: int = 1):
+        """Test / debug surface (ns_llama_set_tap): from now on every eval copies `layer`'s q | k | v before RoPE and its
+        attention output into device buffers of max_rows rows, read back with tap(m).  layer < 0 removes the tap."""
+        import torch
+        E, kvd, _ = self._dims()
+        if layer < 0:
+            _check(lib().ns_llama_set_tap(self.h, -1, None, None, 0), "ns_llama_set_tap")
+            self._tap = None
+            return
+        qkv = torch.empty(max_rows * (E + 2 * kvd), dtype=torch.float32, device="cuda")
+        attn = torch.empty(max_rows * E, dtype=torch.float32, device="cuda")
+        torch.cuda.synchronize()
+        _check(lib().ns_llama_set_tap(self.h, layer, qkv.data_ptr(), attn.data_ptr(), max_rows), "ns_llama_set_tap")
+        self._tap = (qkv, attn)
+
+    def tap(self, m: int):
+        """(q [m, n_embd], k [m, kvd], v [m, kvd], attn [m, n_embd]) of the last eval of m tokens: views of the tap buffers"""
+        E, kvd, _ = self._dims()
+        qkv, attn = self._tap
+        q = qkv[:m * E].view(m, E)
+        k = qkv[m * E:m * (E + kvd)].view(m, kvd)
+        v = qkv[m * (E + kvd):m * (E + 2 * kvd)].view(m, kvd)
+        return q, k, v, attn[:m * E].view(m, E)
+
+    def kv_cache(self, layer: int):
+        """(K, V) fp16 caches of `layer`, each a torch view [n_head_kv, n_ctx, head size] of the engine's device memory"""
+        import torch
+        k, v = C.c_void_p(), C.c_void_p()
+        _check(lib().ns_llama_kv_cache(self.h, layer, C.byref(k), C.byref(v)), "ns_llama_kv_cache")
+        shape = (self.hp.n_head_kv, self.hp.n_ctx, self._dims()[2])
+
+        class _View:  # __cuda_array_interface__ over memory the context owns (valid until close())
+            def __init__(self, ptr):
+                self.__cuda_array_interface__ = dict(shape=shape, typestr="<f2", data=(ptr, False), version=2, strides=None)
+
+        return tuple(torch.as_tensor(_View(p.value), device="cuda") for p in (k, v))
 
     def set_exact_prefill(self, on: bool = True):
         """prompts longer than 32 tokens in pieces of 32: the reference's integer block sums instead of the bf16 tensor-core GEMM"""

@@ -869,6 +869,9 @@ struct ns_llama {
   size_t ws_bytes = 0;
   cudaGraphExec_t decode_exec = nullptr;
   cudaGraph_t decode_graph = nullptr;
+  int tap_layer = -1;  // ns_llama_set_tap: copies of this layer's q|k|v (before RoPE) and attention output
+  float *tap_qkv = nullptr, *tap_attn = nullptr;
+  int tap_rows = 0;
   int* h_state = nullptr;  // pinned host staging
   float* h_logits = nullptr;
 };
@@ -892,6 +895,15 @@ static void dev_free(ns_llama* c, void* p) {
       cudaFree(p);
       return;
     }
+}
+
+// the captured one-token graph bakes in pointers and the enqueued work: rebuilt at the next one-token eval
+static void drop_decode_graph(ns_llama* c) {
+  if (!c->decode_exec) return;
+  cudaGraphExecDestroy(c->decode_exec);
+  cudaGraphDestroy(c->decode_graph);
+  c->decode_exec = nullptr;
+  c->decode_graph = nullptr;
 }
 
 extern "C" ns_llama* ns_llama_create(const ns_llama_hparams* hp, void* queue) {
@@ -976,12 +988,7 @@ extern "C" int ns_llama_set_f32(ns_llama* c, int tensor, int layer, const float*
                        : tensor == NS_LT_ATTN_NORM ? &c->layers[layer].attn_norm
                                                    : &c->layers[layer].ffn_norm;
   if (*slot) {  // set twice: the captured decode graph holds the old pointer
-    if (c->decode_exec) {
-      cudaGraphExecDestroy(c->decode_exec);
-      cudaGraphDestroy(c->decode_graph);
-      c->decode_exec = nullptr;
-      c->decode_graph = nullptr;
-    }
+    drop_decode_graph(c);
     dev_free(c, (void*)*slot);
   }
   *slot = d;
@@ -1014,12 +1021,7 @@ extern "C" int ns_llama_set_weight(ns_llama* c, int tensor, int layer, const ns_
                            : tensor == NS_LT_WO ? &l.wo : tensor == NS_LT_W1 ? &l.w1 : tensor == NS_LT_W2 ? &l.w2 : &l.w3;
     *slot = w;
   }
-  if (c->decode_exec) {  // weights changed: the captured graph holds stale pointers
-    cudaGraphExecDestroy(c->decode_exec);
-    cudaGraphDestroy(c->decode_graph);
-    c->decode_exec = nullptr;
-    c->decode_graph = nullptr;
-  }
+  drop_decode_graph(c);  // weights changed: the captured graph holds stale pointers
   return NS_OK;
 }
 
@@ -1064,12 +1066,7 @@ static int ensure_buffers(ns_llama* c, int m) {
   c->ws_bytes = wsb;
   if (!c->x || !c->xn || !c->qkv || !c->attn || !c->tmp || !c->ws) return NS_E_CUDA;
   c->m_cap = m;
-  if (c->decode_exec) {
-    cudaGraphExecDestroy(c->decode_exec);
-    cudaGraphDestroy(c->decode_graph);
-    c->decode_exec = nullptr;
-    c->decode_graph = nullptr;
-  }
+  drop_decode_graph(c);
   return NS_OK;
 }
 
@@ -1159,6 +1156,9 @@ static int enqueue_forward(ns_llama* c, int m, bool from_state, int advance, int
         if (int rc = ns_mul_mat(L.wv, c->xn, E, v, kvd, m, nullptr, nullptr, 0, c->ws, (void*)st)) return rc;
       }
     }
+    const bool tap = il == c->tap_layer;
+    if (tap)  // before any RoPE: rope_kv_kernel rotates q in place
+      NS_CUDA_TRY(cudaMemcpyAsync(c->tap_qkv, c->qkv, (size_t)m * (E + 2 * kvd) * 4, cudaMemcpyDeviceToDevice, st));
     const bool fast = (hd == 128 || hd == 64);
     static const int dbg_skip = getenv("NS_LLAMA_DEBUG_SKIP") ? atoi(getenv("NS_LLAMA_DEBUG_SKIP")) : 0;  // timing experiments only
     if (m == 1 && (dbg_skip & 1)) {
@@ -1206,6 +1206,7 @@ static int enqueue_forward(ns_llama* c, int m, bool from_state, int advance, int
       }
       ns_count_launch();
     }
+    if (tap) NS_CUDA_TRY(cudaMemcpyAsync(c->tap_attn, c->attn, (size_t)m * E * 4, cudaMemcpyDeviceToDevice, st));
     // inpFF = wo * attn + inpSA, written over x (every row is read by its own output only after the matmul finished)
     if (int rc = ns_mul_mat_engine(L.wo, c->attn, E, c->xn, E, m, c->x, c->ws, st, nullptr, 0.f)) return rc;
     // xn now holds inpFF; FFN + residual back into x, the FFN RMSNorm folded into the gate/up launch where that is a ring GEMV,
@@ -1271,6 +1272,10 @@ extern "C" int ns_llama_eval(ns_llama* c, const int32_t* tokens, int n_tokens, i
     ns_set_error("ns_llama_eval: invalid arguments (n_tokens=%d n_past=%d n_ctx=%d)", n_tokens, n_past, c ? c->hp.n_ctx : 0);
     return NS_E_INVALID;
   }
+  if (c->tap_layer >= 0 && n_tokens > c->tap_rows) {
+    ns_set_error("ns_llama_eval: %d new tokens, the tap set with ns_llama_set_tap holds %d rows", n_tokens, c->tap_rows);
+    return NS_E_INVALID;
+  }
   if (c->exact_prefill && n_tokens > 32) {
     // parity mode: prompts go through in pieces of <= 32 tokens, which the matmuls run on the integer tensor cores with the
     // reference's exact block sums (causal attention over the fp16 KV cache makes the split invisible to the arithmetic)
@@ -1324,6 +1329,32 @@ extern "C" int ns_llama_generate(ns_llama* c, int32_t first_token, int n_past, i
   for (int i = 0; i < n_new; ++i) NS_CUDA_TRY(cudaGraphLaunch(c->decode_exec, st));
   NS_CUDA_TRY(cudaMemcpyAsync(out_tokens, c->record, (size_t)n_new * sizeof(int), cudaMemcpyDeviceToHost, st));
   NS_CUDA_TRY(cudaStreamSynchronize(st));
+  return NS_OK;
+}
+
+extern "C" int ns_llama_set_tap(ns_llama* c, int layer, float* qkv_dst, float* attn_dst, int max_rows) {
+  if (!c) return NS_E_INVALID;
+  if (layer >= 0 && (layer >= c->hp.n_layer || !qkv_dst || !attn_dst || max_rows <= 0)) {
+    ns_set_error("ns_llama_set_tap: layer %d of %d, max_rows %d", layer, c->hp.n_layer, max_rows);
+    return NS_E_INVALID;
+  }
+  NS_CUDA_TRY(cudaStreamSynchronize(c->st));  // nothing in flight still writes to the previous destinations
+  c->tap_layer = layer < 0 ? -1 : layer;
+  c->tap_qkv = layer < 0 ? nullptr : qkv_dst;
+  c->tap_attn = layer < 0 ? nullptr : attn_dst;
+  c->tap_rows = layer < 0 ? 0 : max_rows;
+  drop_decode_graph(c);  // the copies are (or were) nodes of the captured graph
+  return NS_OK;
+}
+
+extern "C" int ns_llama_kv_cache(const ns_llama* c, int layer, const void** k, const void** v) {
+  if (!c || !k || !v || layer < 0 || layer >= c->hp.n_layer) {
+    ns_set_error("ns_llama_kv_cache: invalid arguments (layer %d)", layer);
+    return NS_E_INVALID;
+  }
+  const size_t per_layer = (size_t)c->hp.n_head_kv * c->hp.n_ctx * (c->hp.n_embd / c->hp.n_head);
+  *k = c->kc + (size_t)layer * per_layer;
+  *v = c->vc + (size_t)layer * per_layer;
   return NS_OK;
 }
 

@@ -93,6 +93,16 @@ def soft_max_f16table(s):
     return (e * np.float32(1.0 / np.float64(e.astype(np.float64).sum()))).astype(np.float32)
 
 
+def attention(k, v, q, scale):
+    """One (token, head) of the ggml attention, llama.cpp:286-302: K.Q with Q rounded to fp16 (mul_mat(K fp16, Q)), times
+    scale (ne_scale), soft_max through the fp16 exp table, then V.P with P rounded to fp16 (mul_mat(V fp16, P); the reference
+    keeps V transposed).  k, v [len, hd] hold the fp16 cache rows 0 .. pos (the causal window), q [hd] is rotated."""
+    s = vec_dot_f16_rows(np.asarray(k, np.float32), _f16(q)) * np.float32(scale)
+    p = soft_max_f16table(s)
+    vt = np.ascontiguousarray(np.asarray(v, np.float32).T)
+    return vec_dot_f16_rows(vt, _f16(p))
+
+
 def rms_norm(x, eps):
     """kernel_ref.h:2199-2225 (simplified layernorm without scale): sequential fp32 sum of squares, sqrt, reciprocal"""
     x = np.asarray(x, np.float32)
@@ -153,11 +163,7 @@ class OracleLlama:
                 ln = n_past + t + 1
                 for h in range(H):
                     hk = h // (H // HK)
-                    kk = self.kc[il, hk, :ln].astype(np.float32)              # [ln, hd]
-                    s = vec_dot_f16_rows(kk, _f16(q[t, h])) * scale           # mul_mat(K fp16, Q -> fp16), then ne_scale
-                    p = soft_max_f16table(s)
-                    vt = np.ascontiguousarray(self.vc[il, hk, :ln].astype(np.float32).T)   # the reference keeps V transposed
-                    attn[t, h] = vec_dot_f16_rows(vt, _f16(p))                # mul_mat(V fp16, P -> fp16)
+                    attn[t, h] = attention(self.kc[il, hk, :ln], self.vc[il, hk, :ln], q[t, h], scale)
             inp_ff = self._mm(L["wo"], attn.reshape(n, E)) + x
             cur = self._rms(inp_ff, L["ffn_norm"])
             g = self._mm(L["w1"], cur)

@@ -300,7 +300,8 @@ def test_tensor_core_prompt_attention_against_the_cpu_graph():
 def test_split_context_decode_attention_matches_the_single_cta_kernel(n_head, n_head_kv, monkeypatch):
     """decode attention with K / V staged by TMA and the context split into ranges of 256 positions (attn_decode_kernel) against the
     one-CTA-per-head kernel with dependent row loads (NS_ATTN_OLD_DECODE=1), token by token across the 256 and 512 boundaries
-    (1, 2 and 3 active ranges; a range holding only the new token), head sizes 64 and 128, GQA; smooth fp32-compute engine"""
+    (1, 2 and 3 active ranges; a range holding only the new token), head sizes 64 and 128, GQA; smooth fp32-compute engine.  Past
+    512: three single-token evals, two consecutive generate calls, and an eval that attends to the rows those calls wrote"""
     rng = np.random.default_rng(5)
     prompt = [int(t) for t in rng.integers(3, 320, 250)]
     steps = [int(t) for t in rng.integers(3, 320, 12)]
@@ -317,7 +318,14 @@ def test_split_context_decode_attention_matches_the_single_cta_kernel(n_head, n_
             n_past += 1
         outs.append(eng.eval(jump, n_past)[0])  # to position 512
         n_past += len(jump)
-        gen = eng.generate(7, n_past, 6)        # three ranges, through the decode graph
+        for t in steps[:3]:                     # positions 512 .. 514: three active ranges
+            outs.append(eng.eval([t], n_past)[0])
+            n_past += 1
+        gen = []
+        for first in (7, 8):                    # two consecutive generate calls (graph replays, merge ticket reset between)
+            gen.append(eng.generate(first, n_past, 4))
+            n_past += 4
+        outs.append(eng.eval([9], n_past)[0])   # attends to the K / V rows the generated steps wrote
         eng.close()
         if old:
             monkeypatch.delenv("NS_ATTN_OLD_DECODE")
@@ -325,10 +333,12 @@ def test_split_context_decode_attention_matches_the_single_cta_kernel(n_head, n_
 
     a, ga = run(False)
     b, gb = run(True)
-    for i, (x, y) in enumerate(zip(a, b)):
+    assert len(a) == len(b) == 1 + len(steps) + 1 + 3 + 1
+    same_ids = all(np.array_equal(x, y) for x, y in zip(ga, gb))  # else the last eval attends to different tokens' rows
+    for i, (x, y) in enumerate(zip(a, b) if same_ids else zip(a[:-1], b[:-1])):
         assert np.isfinite(x).all()
         assert float(np.abs(x - y).max()) <= 1e-2 * max(1.0, float(np.abs(y).max())), (i, float(np.abs(x - y).max()))
-    assert len(ga) == 6 and len(gb) == 6  # (greedy ids may part at a near-tie; the logits above are the check)
+    assert [len(g) for g in ga] == [len(g) for g in gb] == [4, 4]  # (greedy ids may part at a near-tie; the logits are the check)
 
 
 def test_long_context_decode_against_the_cpu_graph():

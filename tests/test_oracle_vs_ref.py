@@ -166,21 +166,34 @@ def _vp(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
-@pytest.mark.parametrize("hd", [64, 128])
-def test_llama_rope_mode0_bit_exact(hd):
+@pytest.mark.parametrize("hd,theta,scale", [pytest.param(64, 10000.0, 1.0, id="64"), pytest.param(128, 10000.0, 1.0, id="128"),
+                                            pytest.param(128, 500000.0, 1.0, id="128-theta5e5"),   # Llama-3
+                                            pytest.param(128, 1e6, 1.0, id="128-theta1e6"),
+                                            pytest.param(128, 10000.0, 4.0, id="128-scale4"),
+                                            pytest.param(128, 500000.0, 4.0, id="128-theta5e5-scale4")])
+def test_llama_rope_mode0_bit_exact(hd, theta, scale):
+    """freq_base and freq_scale as hparams hold them (llama.cpp:243-244), at positions up to 4095"""
     from oracle import llama_model as lm
     r = _rng(31)
+    default = (theta, scale) == (10000.0, 1.0)
+    key = f"rope[{hd}]" if default else f"rope[{hd}-{theta:g}-{scale:g}]"
+
     def rope(x, n_tok, n_past):
         y = x.copy().reshape(n_tok, 3, hd)
-        oracle.ref_ne().ref_ne_rope(_vp(y), hd, 3, n_tok, n_past, 10000.0, 1.0)
+        oracle.ref_ne().ref_ne_rope(_vp(y), hd, 3, n_tok, n_past, theta, scale)
         return y
 
     for pos in (0, 1, 7, 33, 127, 2047):
         x = r.normal(0, 1, (3, hd)).astype(np.float32)
-        golden.check(f"rope[{hd}].pos{pos}", lm.rope_mode0(x, pos, hd), lambda: rope(x, 1, pos)[0])
+        golden.check(f"{key}.pos{pos}", lm.rope_mode0(x, pos, hd, theta, scale), lambda: rope(x, 1, pos)[0])
     # several tokens in one call: position n_past + t
     x = r.normal(0, 1, (2, 3, hd)).astype(np.float32)
-    golden.check(f"rope[{hd}].two_tokens", np.stack([lm.rope_mode0(x[t], 10 + t, hd) for t in range(2)]), lambda: rope(x, 2, 10))
+    golden.check(f"{key}.two_tokens", np.stack([lm.rope_mode0(x[t], 10 + t, hd, theta, scale) for t in range(2)]),
+                 lambda: rope(x, 2, 10))
+    # long contexts: theta_base *= theta_scale compounds its fp32 roundings, and sin / cos take arguments in the thousands
+    for pos in (3071, 3998, 3999, 4095):
+        x = r.normal(0, 1, (3, hd)).astype(np.float32)
+        golden.check(f"{key}.pos{pos}", lm.rope_mode0(x, pos, hd, theta, scale), lambda: rope(x, 1, pos)[0])
 
 
 def test_llama_softmax_and_rms_norm_bit_exact():
